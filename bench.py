@@ -16,9 +16,12 @@ and processes threads * T env steps per GPU.  `--config` selects the other BASEL
 With --config c2 (the default) and one GPU the line also carries compact results of c3 and c5 under "other_configs"
 (--no-extras skips them).
 
-`value`  : K iterations replayed from inputs already resident in HBM, device-timed with CUDA events, L2 flushed between
-           iterations; the K-step block is repeated until >= 1 s has been timed (`blocks`), `ms_per_step` is the mean.
-`e2e`    : the same iteration driven from HOST buffers (pinned env outputs -> H2D, D2H of train_info) per step, wall clock.
+`value`  : K = --steps iterations replayed from inputs already resident in HBM, each device-timed with its own pair of CUDA
+           events, L2 flushed between iterations; `ms_per_step` is the mean.
+`e2e`    : then K more iterations driven from HOST buffers (pinned env outputs -> H2D, D2H of train_info) per step, wall clock.
+`--dump-outputs DIR` : after the timed iterations, run one more iteration of the timed path from the seeded starting
+           state and write what it hands its caller as DIR/<name>.npy (dump_outputs).  Inputs, initial weights and RNG
+           seeds are fixed, so two builds run with the same arguments can be compared array by array.
 `--impl reference` : the CPU restatement of the reference path (oracle/, see its header) on the host cores.
 """
 import argparse
@@ -279,8 +282,8 @@ class Job:
             self.eng.upload()
 
 
-def run_config(name, a, world, rank, dev, dist, sampler=None, light=False):
-    """Build the workload, time it.  `light`: compact result for "other_configs" (fewer repeats, no phase breakdown)."""
+def run_config(name, a, world, rank, dev, dist, sampler=None):
+    """Build the workload, time a.steps iterations."""
     import torch
     w = workload(name, world)
     cfg = w["cfg"]
@@ -324,35 +327,22 @@ def run_config(name, a, world, rank, dev, dist, sampler=None, light=False):
             info = j.eng.step_e2e()
         return info
 
-    # ---- device-timed resident loop: blocks of exactly K steps, repeated until >= ~1 s is timed ----
+    # ---- device-timed resident loop: exactly K steps, each between its own pair of events ----
     K = a.steps
     W = max(a.warmup, 3)
     for _ in range(W):
         step_resident()
     barrier()
-    t0 = time.perf_counter()
-    step_resident()
-    torch.cuda.synchronize()
-    est = max(time.perf_counter() - t0, 1e-5)
-    blocks = int(min(max(1, round((0.4 if light else 1.0) / (K * est) + 0.5)), 400))
-    if world > 1:
-        tb = torch.tensor([blocks], device=dev)
-        dist.all_reduce(tb, op=dist.ReduceOp.MAX)
-        blocks = int(tb.item())
     if sampler is not None:
         sampler.start()
-    block_ms = []
+    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
     t_wall0 = time.perf_counter()
-    for _ in range(blocks):
-        barrier()
-        evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
-        for s, e in evs:
-            flush.zero_()                                  # L2 flush between timed iterations (outside the events)
-            s.record()
-            step_resident()
-            e.record()
-        barrier()
-        block_ms.append(sum(s.elapsed_time(e) for s, e in evs))
+    for s, e in evs:
+        flush.zero_()                                      # L2 flush between timed iterations (outside the events)
+        s.record()
+        step_resident()
+        e.record()
+    barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = sum(j.eng.launches_per_iteration for j in jobs) * K
 
@@ -361,38 +351,70 @@ def run_config(name, a, world, rank, dev, dist, sampler=None, light=False):
     prefetch = all([j.eng.enable_input_prefetch() for j in jobs]) if not getattr(a, "no_prefetch", False) else False
     for _ in range(3):
         step_e2e()
-    e2e_blocks = max(1, min(blocks, int(round((0.3 if light else 1.0) / (K * est) + 0.5))))
-    if world > 1:
-        tb = torch.tensor([e2e_blocks], device=dev)
-        dist.all_reduce(tb, op=dist.ReduceOp.MAX)
-        e2e_blocks = int(tb.item())
-    e2e_block_s = []
     info = None
-    for _ in range(e2e_blocks):
-        barrier()
-        t0 = time.perf_counter()
-        for _ in range(K):
-            flush.zero_()
-            info = step_e2e()
-        barrier()
-        e2e_block_s.append(time.perf_counter() - t0)
+    barrier()
+    t0 = time.perf_counter()
+    for _ in range(K):
+        flush.zero_()
+        info = step_e2e()
+    barrier()
+    e2e_s = time.perf_counter() - t0
     clocks = sampler.stop() if sampler is not None else None
 
-    # max over ranks of every block, then the mean over blocks
-    t = torch.tensor(block_ms + [x * 1e3 for x in e2e_block_s], dtype=torch.float64, device=dev)
+    # max over ranks of every step (and of the e2e loop), then the mean over steps
+    t = torch.tensor([s.elapsed_time(e) for s, e in evs] + [e2e_s * 1e3], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     t = t.tolist()
-    bm, em = t[:blocks], t[blocks:]
-    ms_step = sum(bm) / (blocks * K)
-    e2e_ms_step = sum(em) / (len(em) * K)
+    sm = t[:K]
+    ms_step = sum(sm) / K
+    e2e_ms_step = t[K] / K
     steps_env = cfg.n_rollout_threads * cfg.episode_length * world
     res = {"workload": w, "cfg": cfg, "jobs": jobs, "graph_ok": graph_ok, "ms_per_step": ms_step, "value": steps_env / (ms_step * 1e-3),
-           "e2e_ms_per_step": e2e_ms_step, "e2e_value": steps_env / (e2e_ms_step * 1e-3), "blocks": blocks, "e2e_blocks": len(em),
-           "block_ms_per_step": {"min": min(bm) / K, "median": sorted(bm)[len(bm) // 2] / K, "max": max(bm) / K},
+           "e2e_ms_per_step": e2e_ms_step, "e2e_value": steps_env / (e2e_ms_step * 1e-3),
+           "step_ms": {"min": min(sm), "median": sorted(sm)[K // 2], "max": max(sm)},
            "launches": launches, "h2d": sum(j.eng.h2d_bytes() for j in jobs), "d2h": 48 * len(jobs), "clocks": clocks,
            "wall_s_timed_region": t_wall, "info": info, "flush": flush, "steps_env": steps_env, "prefetch": bool(prefetch)}
     return res
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(w, a, rank, dev, out_dir):
+    """One iteration of the timed path (engine.launch_iteration, the launch sequence its CUDA graph replays) from the seeded
+    starting state of the timed jobs -- same initial weights, staged inputs and RNG seeds -- and DIR/<name>.npy of what it
+    hands its caller, per policy (prefix `policy<i>_` when there are several): train_info (float64, engine.INFO_KEYS
+    order), the trained actor / critic parameter vectors, the value normaliser's state, and the rollout storage the
+    iteration filled (actions, log-probs, value predictions, returns, advantages).
+    Not the last timed iteration itself: float atomics in the update sum in a different order from run to run, and over
+    tens of iterations the sampled actions turn those last-bit differences into different trajectories."""
+    import numpy as np
+    import torch
+    jobs = [Job(w, i, dev, rank, a) for i in range(w["n_policies"])]
+    for j in jobs:
+        j.eng.step_resident()                              # no graph captured: launch_iteration()
+    torch.cuda.synchronize()
+    if rank != 0:
+        return
+    arrays = {}
+    for i, j in enumerate(jobs):
+        pre = f"policy{i}_" if len(jobs) > 1 else ""
+        n = j.trainer.ppo_epoch * j.trainer.num_mini_batch
+        arrays[pre + "train_info"] = (j.eng.loss_out / n).cpu().numpy()
+        arrays[pre + "actor_params"] = j.policy.actor.flat
+        arrays[pre + "critic_params"] = j.policy.critic.flat
+        if j.trainer.value_normalizer is not None:
+            arrays[pre + "value_normalizer"] = j.trainer.value_normalizer.state
+        for k in ("actions", "action_log_probs", "value_preds", "returns", "advantages"):
+            arrays[pre + k] = getattr(j.buf, k)
+    arrays = {k: v if isinstance(v, np.ndarray) else v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def kernel_roofline(res, a, peaks, tf32_peak):
@@ -595,7 +617,7 @@ def result_line(name, res, a, world, roof, cpu, clocks, extra_cfg):
                        "h2d": "obs, rewards, dones (share_obs = concat of the thread's agents' obs is formed on the device)"
                               if eng.share_from_obs else "obs, share_obs, rewards, dones (+ active / avail masks)",
                        **extra_cfg},
-            "timing": {"blocks_of_k_steps": res["blocks"], "block_ms_per_step": res["block_ms_per_step"], "e2e_blocks": res["e2e_blocks"],
+            "timing": {"timed_steps": a.steps, "step_ms": res["step_ms"], "e2e_timed_steps": a.steps,
                        "wall_s_timed_region": res["wall_s_timed_region"]},
             "e2e": {"value": res["e2e_value"], "unit": UNIT, "h2d_bytes_per_step": res["h2d"], "d2h_bytes_per_step": res["d2h"],
                     "ms_per_step": res["e2e_ms_per_step"],
@@ -635,6 +657,8 @@ def run_gpu(a):
 
     sampler = ClockSampler(local)
     res = run_config(a.config, a, world, rank, dev, dist, sampler)
+    if a.dump_outputs:
+        dump_outputs(res["workload"], a, rank, dev, a.dump_outputs)
     cfg = res["cfg"]
     eng0 = res["jobs"][0].eng
 
@@ -707,7 +731,7 @@ def run_gpu(a):
             if a.gemm == "tf32" and a.config in ("c2", "c5"):
                 try:
                     a2 = argparse.Namespace(**{**vars(a), "gemm": "fp32", "steps": max(3, a.steps // 4)})
-                    r2 = run_config(a.config, a2, 1, 0, dev, dist, None, light=True)
+                    r2 = run_config(a.config, a2, 1, 0, dev, dist, None)
                     line["value_fp32"] = {"value": r2["value"], "ms_per_step": r2["ms_per_step"], "e2e_value": r2["e2e_value"],
                                           "gemm": "fp32 (exact FFMA build of the same kernels)"}
                     del r2
@@ -717,7 +741,7 @@ def run_gpu(a):
             for other in (["c3", "c5"] if a.config == "c2" else []):
                 try:
                     a3 = argparse.Namespace(**{**vars(a), "steps": 3 if other == "c5" else max(3, a.steps // 4), "env": "staged"})
-                    r3 = run_config(other, a3, 1, 0, dev, dist, None, light=True)
+                    r3 = run_config(other, a3, 1, 0, dev, dist, None)
                     rf = kernel_roofline(r3, a3, peaks, tf32_peak)
                     c3, _ = cpu_baseline(other, {"c3": 3, "c5": 2}[other]) if a.cpu_iters > 0 else (None, None)
                     ol = result_line(other, r3, a3, 1, rf, c3, None, {})
@@ -739,7 +763,8 @@ def run_gpu(a):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed iterations (default 50; 5 for c4 and 10 for c5, ~0.1 - 0.5 s per iteration)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c2", choices=["c2", "c3", "c4", "c5"], help="BASELINE.json workload (default c2 = configs[1])")
@@ -753,9 +778,12 @@ def main():
     ap.add_argument("--cpu-iters", type=int, default=100, help="oracle iterations for cpu_baseline (rank 0, N=1); 0 = skip")
     ap.add_argument("--no-extras", dest="extras", action="store_false", help="skip value_fp32 / other_configs")
     ap.add_argument("--no-breakdown", dest="breakdown", action="store_false")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after timing, write the outputs of one iteration from the seeded starting state as DIR/<name>.npy")
     a = ap.parse_args()
-    if a.config in ("c4", "c5") and a.steps > 10:
-        a.steps = 10 if a.config == "c5" else 5             # ~0.1 - 0.5 s per iteration: keep the default run in minutes
+    if a.steps is None:
+        a.steps = {"c4": 5, "c5": 10}.get(a.config, 50)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
         run_reference(a)
     else:
