@@ -413,6 +413,13 @@ static int device_sm_count() {
   return v;
 }
 
+// A net that qualifies for a warp-per-row kernel has its image packed in that kernel's layout (pack_rollout_launch), and
+// that image can be smaller than the tile layout.  When the OTHER net sends both onto the 32-row tile kernels, such a net
+// loads its weights from the flat parameters instead.
+static inline const float* tile_image(const NetDev& n, const float* image) {
+  return (fast_rollout_supported(n) || gru_fast_supported(n)) ? nullptr : image;
+}
+
 int policy_step_launch(const NetDev* na, const NetDev* nc, const PolArgs& a, cudaStream_t st) {
   const NetDev& ref = na ? *na : *nc;
   {   // feed-forward nets with a packed image: the warp-per-two-rows path (rollout_mlp.cuh)
@@ -474,6 +481,11 @@ int policy_step_launch(const NetDev* na, const NetDev* nc, const PolArgs& a, cud
     bytes = b > bytes ? b : bytes;
   }
   if (bytes > 227 * 1024) { set_error("policy_step: %zu B shared memory per CTA > 227 KB (in_dim too large)", bytes); return MAPPO_ERR_UNSUPPORTED; }
+  PolArgs ta = a;
+  for (int w = 0; w < 2; ++w) {
+    const NetDev* n = w == 0 ? na : nc;
+    if (n) ta.image[w] = tile_image(*n, ta.image[w]);
+  }
   auto kern = policy_step_kernel<4>;
   static thread_local SmemConfig configured_dev = {};
   size_t& configured = configured_dev.slot();
@@ -483,7 +495,7 @@ int policy_step_launch(const NetDev* na, const NetDev* nc, const PolArgs& a, cud
     configured = bytes;
   }
   const dim3 grid((a.n_rows + kPolTR - 1) / kPolTR, (na && nc) ? 2 : 1);
-  kern<<<grid, 4 * kPolTR, bytes, st>>>(na ? *na : ref, nc ? *nc : ref, a, na ? 0 : 1);
+  kern<<<grid, 4 * kPolTR, bytes, st>>>(na ? *na : ref, nc ? *nc : ref, ta, na ? 0 : 1);
   return check_launch("policy_step_kernel");
 }
 
@@ -526,6 +538,9 @@ int rollout_persistent_launch(const NetDev& na, const NetDev& nc, const RolloutA
     bytes = b > bytes ? b : bytes;
   }
   if (bytes > 227 * 1024) { set_error("rollout: %zu B shared memory per CTA > 227 KB", bytes); return MAPPO_ERR_UNSUPPORTED; }
+  RolloutArgs ta = a;
+  ta.image[0] = tile_image(na, a.image[0]);
+  ta.image[1] = tile_image(nc, a.image[1]);
   auto kern = rollout_persistent_kernel<4>;
   static thread_local SmemConfig configured_dev = {};
   size_t& configured = configured_dev.slot();
@@ -535,7 +550,7 @@ int rollout_persistent_launch(const NetDev& na, const NetDev& nc, const RolloutA
     configured = bytes;
   }
   const dim3 grid((a.E + kPolTR - 1) / kPolTR, 2);
-  kern<<<grid, 4 * kPolTR, bytes, st>>>(na, nc, a);
+  kern<<<grid, 4 * kPolTR, bytes, st>>>(na, nc, ta);
   return check_launch("rollout_persistent_kernel");
 }
 

@@ -196,6 +196,8 @@ int update_mlp_launch(const NetDev& n, const float* params, const BatchDev& b, c
   if (n.head_total > 32) { set_error("update_mlp: sum(head_dim)=%d > 32", n.head_total); return MAPPO_ERR_UNSUPPORTED; }
   if (n.in_dim <= 64)
     return launch_upd<4>(n, params, b, L, norm_stats, adv_stats, vn_state, grad_part, n_slots, loss_out, feat_out, dfeat_in, st);
+  // <64, 4, 8> is instantiated for inputs up to 128, but its 64-row tiles fit in 227 KB of shared memory only up to in_dim 96
+  // (layer_N 1): from 97 the shared-memory check in launch_upd refuses the net before launching
   if (n.in_dim <= 128)
     return launch_upd<8>(n, params, b, L, norm_stats, adv_stats, vn_state, grad_part, n_slots, loss_out, feat_out, dfeat_in, st);
   set_error("update_mlp: in_dim %d > 128 not built in the fused SIMT path", n.in_dim);

@@ -60,6 +60,14 @@ class SegmentedGraph:
 INFO_KEYS = ("value_loss", "policy_loss", "dist_entropy", "actor_grad_norm", "critic_grad_norm", "ratio")
 
 
+def warp_per_row_rollout(*descs) -> bool:
+    """True when every net qualifies for the warp-per-row rollout kernels: hidden 64, in_dim <= 64 and at most 32 head
+    outputs (csrc/rollout_mlp.cuh fast_rollout_supported, csrc/rollout_gru.cuh gru_fast_supported).  The persistent
+    rollout takes that path only when BOTH nets qualify; otherwise it runs the 32-row tile kernels, which read share_obs
+    from its own staging buffer, and mappo_rollout_closed_loop is not built at all."""
+    return all(d.hidden == 64 and d.in_dim <= 64 and sum(d.head_dim[k] for k in range(d.n_heads)) <= 32 for d in descs)
+
+
 class RolloutEngine:
     def __init__(self, args, policy, trainer, buffer, rng: str = "device", seed: int = 1,
                  share_obs_from_obs: bool = False, device_env=None):
@@ -94,12 +102,15 @@ class RolloutEngine:
                 raise NotImplementedError("closed-loop device env with hidden >= 128 nets")
             want_persistent = False
         self.persistent_rollout = want_persistent and device_env is None
-        # closed loop as ONE launch (mappo_rollout_closed_loop): feed-forward policies
-        self.closed_persistent = want_persistent and device_env is not None and not self.recurrent
+        # closed loop as ONE launch (mappo_rollout_closed_loop): feed-forward policies whose nets both take the warp-per-row
+        # path (a wider critic, e.g. 4-agent simple_spread's share_obs of 96, steps the env per step instead)
+        fast = warp_per_row_rollout(policy.actor.desc, policy.critic.desc)
+        self.closed_persistent = want_persistent and device_env is not None and not self.recurrent and fast
         if device_env is not None and (device_env.N * device_env.M != E or device_env.obs_dim != self.Do
                                        or device_env.share_dim != self.Ds):
             raise ValueError("device_env does not match the rollout storage (rows / obs_dim / share_obs_dim)")
-        self.share_from_obs = bool(share_obs_from_obs) and self.persistent_rollout and not self.recurrent \
+        # (wider nets stage share_obs like any other input)
+        self.share_from_obs = bool(share_obs_from_obs) and self.persistent_rollout and not self.recurrent and fast \
             and self.Ds % self.Do == 0 and E % (self.Ds // self.Do) == 0
         # device staging of one iteration of env outputs (next obs for slots 1..T, rewards, dones, ...): ONE flat buffer
         # (= one H2D copy per iteration) with views per field

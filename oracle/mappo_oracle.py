@@ -482,7 +482,7 @@ def actor_evaluate(cfg, p, obs, hxs, actions, masks, avail=None, active=None):
 # trainer  (algorithms/r_mappo/r_mappo.py)
 # --------------------------------------------------------------------------------------------
 def _huber(e, d):                                                                 # utils/util.py:23-26
-    a = (e.abs() <= d).float()
+    a = (e.abs() <= d).to(e.dtype)
     return a * e ** 2 / 2 + (1 - a) * d * (e.abs() - d / 2)
 
 
@@ -490,11 +490,14 @@ class Learner:
     """Actor + critic parameter sets, two Adam optimisers (rMAPPOPolicy.py:31-37), ValueNorm,
     and the reference update rule (r_mappo.py:52-224)."""
 
-    def __init__(self, cfg: PathConfig, actor: Dict[str, torch.Tensor], critic: Dict[str, torch.Tensor], happo: bool = False):
+    def __init__(self, cfg: PathConfig, actor: Dict[str, torch.Tensor], critic: Dict[str, torch.Tensor], happo: bool = False,
+                 dtype: torch.dtype = torch.float32):
+        """`dtype`: parameters and inputs are cast to it (float64 gives a high-precision reference of the same update)."""
         self.cfg = cfg
+        self.dtype = dtype
         self.happo = happo            # algorithms/happo/happo_trainer.py instead of r_mappo.py (see ppo_update / train)
-        self.actor = {k: v.detach().clone().float().requires_grad_(True) for k, v in actor.items()}
-        self.critic = {k: v.detach().clone().float().requires_grad_(True) for k, v in critic.items()}
+        self.actor = {k: v.detach().clone().to(dtype).requires_grad_(True) for k, v in actor.items()}
+        self.critic = {k: v.detach().clone().to(dtype).requires_grad_(True) for k, v in critic.items()}
         self.opt_a = torch.optim.Adam(list(self.actor.values()), lr=cfg.lr, eps=cfg.opti_eps, weight_decay=0)
         self.opt_c = torch.optim.Adam(list(self.critic.values()), lr=cfg.critic_lr, eps=cfg.opti_eps,
                                       weight_decay=0)
@@ -503,21 +506,21 @@ class Learner:
     # ---- rollout side (rMAPPOPolicy.py:48-86) ----
     @torch.no_grad()
     def get_actions(self, share_obs, obs, h_a, h_c, masks, avail=None, deterministic=False, exp_noise=None):
-        t = lambda a: None if a is None else torch.as_tensor(np.asarray(a), dtype=torch.float32)
+        t = lambda a: None if a is None else torch.as_tensor(np.asarray(a), dtype=self.dtype)
         acts, lps, h_a2 = actor_act(self.cfg, self.actor, t(obs), t(h_a), t(masks), t(avail), deterministic,
-                                    None if exp_noise is None else torch.as_tensor(exp_noise))
+                                    None if exp_noise is None else torch.as_tensor(exp_noise, dtype=self.dtype))
         vals, h_c2 = critic_forward(self.cfg, self.critic, t(share_obs), t(h_c), t(masks))
         return vals, acts, lps, h_a2, h_c2
 
     @torch.no_grad()
     def get_values(self, share_obs, h_c, masks):
-        t = lambda a: torch.as_tensor(np.asarray(a), dtype=torch.float32)
+        t = lambda a: torch.as_tensor(np.asarray(a), dtype=self.dtype)
         return critic_forward(self.cfg, self.critic, t(share_obs), t(h_c), t(masks))[0]
 
     # ---- one optimiser step (r_mappo.py:91-169) ----
     def ppo_update(self, sample, update_actor=True, keep_grads=False):
         c = self.cfg
-        t = lambda a: None if a is None else torch.as_tensor(np.asarray(a), dtype=torch.float32)
+        t = lambda a: None if a is None else torch.as_tensor(np.asarray(a), dtype=self.dtype)
         (share_obs, obs, h_a, h_c, actions, v_old, ret, masks, active, lp_old, adv, avail) = map(t, sample[:12])
 
         values, _ = critic_forward(c, self.critic, share_obs, h_c, masks)

@@ -121,3 +121,20 @@ def grad_agreement(got, want, key, smooth, tf32, report=None, l2_tol=None):
         report.append(f"{key}: max err / scale {err.max() / scale:.3e}, rel L2 {l2:.3e}, outside element tolerance {100 * outside:.2f} %"
                       + ("" if ok else "  <-- FAIL"))
     return ok, l2
+
+
+def rollout_image_floats(in_dim, layer_n, use_fn, recurrent, head_total, hidden=64):
+    """(warp-per-row image, 32-row tile image) sizes in floats of a hidden-64 net's rollout weights: the layouts of
+    csrc/rollout_mlp.cuh make_fast_img (+ rollout_gru.cuh make_gru_fast_img) and csrc/common.cuh make_smem_w."""
+    H = hidden
+    k1 = (in_dim + 3) & ~3
+    ap = (head_total + 3) & ~3
+    fast = (2 * k1 if use_fn else 0) + k1 * H + 3 * H + layer_n * (H * H + 3 * H) + H * ap + ap
+    if recurrent:
+        fast += 2 * 3 * H * H + 2 * 3 * H + 2 * H
+    ld1, ldh = in_dim | 1, H | 1
+    tile = (2 * in_dim if use_fn else 0) + H * ld1 + 3 * H + layer_n * (H * ldh + 3 * H)
+    if recurrent:
+        tile += 2 * 3 * H * ldh + 2 * 3 * H + 2 * H
+    tile += head_total * ldh + head_total
+    return fast, (tile + 3) & ~3

@@ -155,3 +155,47 @@ def test_chunk_rows_oracle_straddles_like_reference():
     E = N * M
     assert list(rows[:, 2]) == [t * E + 0 for t in range(20, 25)] + [t * E + 1 for t in range(0, 5)]
     assert first[2] == 20 * E
+
+
+@pytest.mark.parametrize("recurrent", [0, 1])
+def test_hidden64_dispatch_limits_at_widths_63_to_128(recurrent):
+    """Which kernel family a hidden-64 net gets is decided by its input width: tf32 updates up to in_dim 63, the warp-per-row
+    rollout image up to 64 and the 32-row tile image from 65 (csrc/rollout_mlp.cuh, rollout_gru.cuh, common.cuh)."""
+    from mappo_b200 import _lib
+    from helpers import rollout_image_floats
+    lib = _lib.load()
+    for in_dim in (63, 64, 65, 128):
+        for layer_n, use_fn, heads in ((1, 1, (5,)), (2, 0, (5, 7)), (1, 1, (1,))):
+            d = _lib.NetDesc()
+            d.in_dim, d.hidden, d.layer_n, d.use_feature_norm, d.use_relu, d.recurrent = in_dim, 64, layer_n, use_fn, 1, recurrent
+            d.n_heads = len(heads)
+            for k, a in enumerate(heads):
+                d.head_dim[k] = a
+            d.is_critic = int(heads == (1,))
+            want_tf32 = int(in_dim <= 63 and layer_n == 1)
+            assert lib.mappo_tf32_supported(C.byref(d)) == want_tf32, (in_dim, layer_n)
+            fast, tile = rollout_image_floats(in_dim, layer_n, use_fn, recurrent, sum(heads))
+            assert fast != tile
+            assert lib.mappo_rollout_image_floats(C.byref(d)) == (fast if in_dim <= 64 else tile), (in_dim, layer_n, heads)
+
+
+def test_engine_takes_the_derived_share_obs_and_closed_loop_only_for_warp_per_row_nets():
+    """mappo_rollout_persistent derives share_obs from obs, and mappo_rollout_closed_loop runs, only when both nets take the
+    warp-per-row kernels; the engine mirrors that rule (a 4-agent simple_spread critic is 96 wide)."""
+    from mappo_b200 import _lib
+    from mappo_b200.engine import warp_per_row_rollout
+
+    def desc(in_dim, hidden=64, heads=(5,)):
+        d = _lib.NetDesc()
+        d.in_dim, d.hidden, d.layer_n, d.n_heads = in_dim, hidden, 1, len(heads)
+        for k, a in enumerate(heads):
+            d.head_dim[k] = a
+        return d
+
+    assert warp_per_row_rollout(desc(18), desc(54, heads=(1,)))                   # 3-agent spread (c1 / c2)
+    assert warp_per_row_rollout(desc(64), desc(64, heads=(1,)))
+    assert not warp_per_row_rollout(desc(24), desc(96, heads=(1,)))               # 4-agent spread: the critic is 96 wide
+    assert not warp_per_row_rollout(desc(65), desc(64, heads=(1,)))
+    assert not warp_per_row_rollout(desc(18, hidden=128), desc(54, hidden=128, heads=(1,)))
+    assert not warp_per_row_rollout(desc(18, heads=(20, 13)), desc(54, heads=(1,)))   # 33 head outputs
+    assert warp_per_row_rollout(desc(18, heads=(20, 12)), desc(54, heads=(1,)))
