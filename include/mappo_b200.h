@@ -175,6 +175,26 @@ int32_t mappo_rollout_closed_loop(const mappo_net_desc_t* actor_desc, const floa
                                   const double* reset_states, uint64_t env_seed, uint64_t* env_counter_dev,
                                   const float* exp_noise, uint64_t rng_seed, uint64_t* rng_offset_dev, int32_t T, int32_t E,
                                   int32_t num_agents, int32_t num_landmarks, int32_t episode_length, void* stream);
+/* The same closed loop for either MPE world and for recurrent policies.  world: MAPPO_WORLD_SPREAD (state and reset_states as
+ * above; goal / comm NULL) or MAPPO_WORLD_REFERENCE (simple_reference, state as in mappo_mpe_reference_step: num_agents 2,
+ * num_landmarks 3, goal / comm [n_envs, 2]; reset_states [T, n_envs, 12]).  The actor must match the world's action space
+ * (Discrete(5) / MultiDiscrete(5, 10)) and observation width, the critic its share_obs width (MAPPO_ERR_INVALID otherwise).
+ * Feed-forward nets: h_actor / h_critic NULL.  Recurrent (GRU) nets: h_actor / h_critic = the rnn-state storage [T + 1, E, hidden]
+ * (slot 0 read; slots 1..T written with the state after step t, zero for rows whose episode ended at step t, as
+ * mappo_policy_step followed by mappo_env_insert leaves them); each world group then runs on a 2-CTA cluster (actor CTA with the
+ * worlds, critic CTA).  Nets off the warp-per-row kernels (hidden 64, in_dim <= 64, <= 32 head outputs) or needing more than
+ * 227 KB of shared memory per CTA: MAPPO_ERR_UNSUPPORTED.  Counters advance as in mappo_rollout_closed_loop. */
+#define MAPPO_WORLD_SPREAD 0
+#define MAPPO_WORLD_REFERENCE 1
+int32_t mappo_rollout_closed_loop_ex(const mappo_net_desc_t* actor_desc, const float* actor_image,
+                                     const mappo_net_desc_t* critic_desc, const float* critic_image, float* obs,
+                                     float* share_obs, float* h_actor, float* h_critic, float* masks, float* value_preds,
+                                     float* actions, float* logp, float* rewards, int32_t world, double* agent_pos,
+                                     double* agent_vel, double* landmark_pos, int32_t* goal, int32_t* comm,
+                                     int32_t* step_count, const double* reset_states, uint64_t env_seed,
+                                     uint64_t* env_counter_dev, const float* exp_noise, uint64_t rng_seed,
+                                     uint64_t* rng_offset_dev, int32_t T, int32_t E, int32_t num_agents,
+                                     int32_t num_landmarks, int32_t episode_length, void* stream);
 int32_t mappo_rollout_image_floats(const mappo_net_desc_t* desc);
 int32_t mappo_pack_rollout_weights(const mappo_net_desc_t* desc, const float* params, float* image, void* stream);
 

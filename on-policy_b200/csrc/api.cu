@@ -309,11 +309,27 @@ int32_t mappo_rollout_closed_loop(const mappo_net_desc_t* ad, const float* a_img
                                   uint64_t* env_counter_dev, const float* exp_noise, uint64_t rng_seed,
                                   uint64_t* rng_offset_dev, int32_t T, int32_t E, int32_t num_agents, int32_t num_landmarks,
                                   int32_t episode_length, void* stream) {
+  return mappo_rollout_closed_loop_ex(ad, a_img, cd, c_img, obs, share_obs, nullptr, nullptr, masks, value_preds, actions, logp,
+                                      rewards, MAPPO_WORLD_SPREAD, agent_pos, agent_vel, landmark_pos, nullptr, nullptr, step_count,
+                                      reset_states, env_seed, env_counter_dev, exp_noise, rng_seed, rng_offset_dev, T, E,
+                                      num_agents, num_landmarks, episode_length, stream);
+}
+
+int32_t mappo_rollout_closed_loop_ex(const mappo_net_desc_t* ad, const float* a_img, const mappo_net_desc_t* cd, const float* c_img,
+                                     float* obs, float* share_obs, float* h_actor, float* h_critic, float* masks, float* value_preds,
+                                     float* actions, float* logp, float* rewards, int32_t world, double* agent_pos,
+                                     double* agent_vel, double* landmark_pos, int32_t* goal, int32_t* comm, int32_t* step_count,
+                                     const double* reset_states, uint64_t env_seed, uint64_t* env_counter_dev,
+                                     const float* exp_noise, uint64_t rng_seed, uint64_t* rng_offset_dev, int32_t T, int32_t E,
+                                     int32_t num_agents, int32_t num_landmarks, int32_t episode_length, void* stream) {
   int rc = validate_desc(ad); if (rc) return rc;
   rc = validate_desc(cd); if (rc) return rc;
   if (ad->is_critic || !cd->is_critic) { set_error("rollout_closed_loop: actor/critic descriptors swapped"); return MAPPO_ERR_INVALID; }
   if (!a_img || !c_img || !obs || !share_obs || !masks || !value_preds || !actions || !logp || !rewards || !agent_pos ||
       !agent_vel || !landmark_pos || !step_count || T <= 0 || E <= 0 || episode_length <= 0) { set_error("rollout_closed_loop: NULL / bad argument"); return MAPPO_ERR_INVALID; }
+  if (world != MAPPO_WORLD_SPREAD && world != MAPPO_WORLD_REFERENCE) { set_error("rollout_closed_loop: unknown world %d", world); return MAPPO_ERR_INVALID; }
+  if (world == MAPPO_WORLD_REFERENCE && (!goal || !comm || num_agents != 2 || num_landmarks != 3)) { set_error("rollout_closed_loop: simple_reference needs goal / comm state, 2 agents and 3 landmarks"); return MAPPO_ERR_INVALID; }
+  if ((ad->recurrent && !h_actor) || (cd->recurrent && !h_critic)) { set_error("rollout_closed_loop: recurrent net without state storage"); return MAPPO_ERR_INVALID; }
   if (!exp_noise && !rng_offset_dev) { set_error("rollout_closed_loop: sampling needs exp_noise or rng_offset_dev"); return MAPPO_ERR_INVALID; }
   if (!reset_states && !env_counter_dev) { set_error("rollout_closed_loop: resets need reset_states or env_counter_dev"); return MAPPO_ERR_INVALID; }
   ClosedArgs ca;
@@ -321,9 +337,11 @@ int32_t mappo_rollout_closed_loop(const mappo_net_desc_t* ad, const float* a_img
   RolloutArgs& a = ca.r;
   a.image[0] = a_img; a.image[1] = c_img;
   a.obs = obs; a.share_obs = share_obs; a.masks = masks; a.value_preds = value_preds; a.actions = actions; a.logp = logp;
+  a.h_actor = ad->recurrent ? h_actor : nullptr; a.h_critic = cd->recurrent ? h_critic : nullptr;
   a.rewards = rewards; a.exp_noise = exp_noise; a.rng_seed = rng_seed; a.rng_offset = rng_offset_dev; a.T = T; a.E = E;
-  ca.apos = agent_pos; ca.avel = agent_vel; ca.lpos = landmark_pos; ca.step_count = step_count; ca.reset_states = reset_states;
-  ca.env_seed = env_seed; ca.env_counter = env_counter_dev; ca.M = num_agents; ca.L = num_landmarks;
+  ca.world = world;
+  ca.apos = agent_pos; ca.avel = agent_vel; ca.lpos = landmark_pos; ca.goal = goal; ca.comm = comm; ca.step_count = step_count;
+  ca.reset_states = reset_states; ca.env_seed = env_seed; ca.env_counter = env_counter_dev; ca.M = num_agents; ca.L = num_landmarks;
   ca.episode_length = episode_length;
   rc = rollout_closed_launch(make_net_dev(ad), make_net_dev(cd), ca, (cudaStream_t)stream);
   if (rc) return rc;

@@ -517,6 +517,26 @@ struct SmemConfig {
   }
 };
 
+// ---- thread-block clusters: barrier and distributed shared memory (DSMEM) -----------------------------------------------------
+__device__ __forceinline__ void cluster_sync_all() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+__device__ __forceinline__ uint32_t cluster_cta_rank() {
+  uint32_t r;
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+  return r;
+}
+// store into the shared memory of CTA `rank` of this cluster, at the address `local` has in this CTA's own window
+__device__ __forceinline__ void st_cluster_f32(const float* local, uint32_t rank, float v) {
+  uint32_t remote;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"((uint32_t)__cvta_generic_to_shared(local)), "r"(rank));
+  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(remote), "f"(v) : "memory");
+}
+// the two halves of a cluster barrier, for threads that have work to do between signalling and waiting (not .aligned: callable
+// where a warp may have diverged); arrive releases and wait acquires this thread's shared / DSMEM writes at cluster scope
+__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive;" ::: "memory"); }
+__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait;" ::: "memory"); }
+
 // ---- programmatic dependent launch (PDL) for the chains of small dependent kernels of an optimiser step -------------------------
 // A kernel launched with launch_pdl() may be SCHEDULED while its stream predecessor still runs: its CTAs take their SMs and park in
 // pdl_prologue() (griddepcontrol.wait) until the predecessor grid has completed and flushed, so the ~2 us of launch / scheduling

@@ -66,12 +66,15 @@ struct MpeRefArgs {                      // `simple_reference`: 2 agents, 3 land
 };
 int mpe_reference_launch(const MpeRefArgs& a, cudaStream_t st);
 
-// closed rollout loop with the device-side simple_spread worlds (rollout_closed.cuh)
+// closed rollout loop with the device-side MPE worlds (rollout_closed.cuh)
 struct ClosedArgs {
-  RolloutArgs r;                     // storage pointers, images, sampling noise / RNG, T, E (f_* unused)
+  RolloutArgs r;                     // storage pointers (h_actor / h_critic: recurrent nets), images, sampling noise / RNG, T, E
+                                     // (f_* unused)
+  int world;                         // MAPPO_WORLD_SPREAD / MAPPO_WORLD_REFERENCE
   double *apos, *avel, *lpos;        // world state [N][M][2], [N][M][2], [N][L][2]
+  int32_t *goal, *comm;              // simple_reference only: [N][2] each (NULL for simple_spread)
   int32_t* step_count;               // [N]
-  const double* reset_states;        // [T][N][2 (M + L)] episode starts to use when a world ends at step t, or NULL (Philox)
+  const double* reset_states;        // [T][N][per-world doubles] episode starts to use when a world ends at step t, or NULL (Philox)
   uint64_t env_seed;
   const uint64_t* env_counter;
   int M, L, episode_length;

@@ -1,4 +1,4 @@
-// mpe_env.cu -- N vectorised MPE `simple_spread` worlds stepped on the device (SURVEY.md section 8(f), row f1).
+// mpe_env.cu -- N vectorised MPE `simple_spread` / `simple_reference` worlds stepped on the device (SURVEY.md section 8(f), row f1).
 //
 // Replaces, for this scenario, SubprocVecEnv.step -> MultiAgentEnv.step -> World.step + the scenario callbacks
 // (envs/env_wrappers.py:140-154, envs/mpe/environment.py:115-146, envs/mpe/core.py:207-323,
@@ -58,86 +58,26 @@ int mpe_spread_launch(const MpeArgs& a, cudaStream_t st) {
   return check_launch("mpe_spread_kernel");
 }
 
-// ---- `simple_reference` (BASELINE configs[2]'s scenario) -------------------------------------------------------------
-// envs/mpe/scenarios/simple_reference.py:8-97: 2 agents, 3 landmarks, 10 communication symbols, nothing collides.  Agent m
-// wants the OTHER agent on landmark goal[m]; both receive r_0 + r_1, r_m = -|pos[1 - m] - landmark[goal_m]|^2 (:62-67 with
-// shared_reward, environment.py:139-142).  Action = MultiDiscrete([[0,4],[0,9]]) (environment.py:55-63): a movement head
-// decoded like simple_spread's and a symbol head that becomes the agent's communication state (core.py:283-290, c_noise
-// None).  Observation (:69-97) = velocity, landmarks - pos, colour of the goal landmark, the other agent's communication.
-constexpr int kRefAgents = 2, kRefLandmarks = 3, kRefSymbols = 10, kRefObs = 2 + 2 * kRefLandmarks + 3 + kRefSymbols;
-
+// ---- `simple_reference` (BASELINE configs[2]'s scenario; the world functions are in mpe_world.cuh) -------------------
 __global__ void __launch_bounds__(128) mpe_reference_kernel(const MpeRefArgs a) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= a.N) return;
-  constexpr int M = kRefAgents, L = kRefLandmarks;
-  double ap[M][2], av[M][2], lp[L][2];
-  int goal[M], comm[M];
-  for (int m = 0; m < M; ++m)
-    for (int d = 0; d < 2; ++d) { ap[m][d] = a.apos[((size_t)e * M + m) * 2 + d]; av[m][d] = a.avel[((size_t)e * M + m) * 2 + d]; }
-  for (int l = 0; l < L; ++l)
-    for (int d = 0; d < 2; ++d) lp[l][d] = a.lpos[((size_t)e * L + l) * 2 + d];
-  for (int m = 0; m < M; ++m) { goal[m] = a.goal[(size_t)e * M + m]; comm[m] = a.comm[(size_t)e * M + m]; }
-  int step = a.step_count[e];
+  constexpr int M = kRefAgents;
+  MpeRefWorld w;
+  ref_world_load(w, a.apos, a.avel, a.lpos, a.goal, a.comm, a.step_count, e);
   double reward = 0.0;
   bool done = false;
   if (a.actions) {
-    for (int m = 0; m < M; ++m) {          // environment.py:184-250 (_set_action), core.py:229-238, :267-281 (no contacts)
-      const int mv = (int)a.actions[((size_t)e * M + m) * 2], sym = (int)a.actions[((size_t)e * M + m) * 2 + 1];
-      double u[2];
-      u[0] = d_mul(d_add(0.0, d_sub(mv == 1 ? 1.0 : 0.0, mv == 2 ? 1.0 : 0.0)), kSensitivity);
-      u[1] = d_mul(d_add(0.0, d_sub(mv == 3 ? 1.0 : 0.0, mv == 4 ? 1.0 : 0.0)), kSensitivity);
-      for (int d = 0; d < 2; ++d) {
-        const double f = d_add(d_mul(1.0, u[d]), 0.0);
-        double v = d_mul(av[m][d], 1 - kDamping);
-        v = d_add(v, d_mul(d_div(f, 1.0), kDt));
-        av[m][d] = v;
-        ap[m][d] = d_add(ap[m][d], d_mul(v, kDt));
-      }
-      comm[m] = sym < 0 ? 0 : (sym >= kRefSymbols ? kRefSymbols - 1 : sym);
-    }
-    step += 1;
-    for (int m = 0; m < M; ++m) {          // simple_reference.py:62-67
-      const double dx = d_sub(ap[1 - m][0], lp[goal[m]][0]), dy = d_sub(ap[1 - m][1], lp[goal[m]][1]);
-      const double r = -d_add(d_mul(dx, dx), d_mul(dy, dy));
-      reward = m == 0 ? r : d_add(reward, r);
-    }
-    done = step >= a.episode_length;
+    int mv[M], sym[M];
+    for (int m = 0; m < M; ++m) { mv[m] = (int)a.actions[((size_t)e * M + m) * 2]; sym[m] = (int)a.actions[((size_t)e * M + m) * 2 + 1]; }
+    reward = ref_world_step(w, mv, sym, a.episode_length, &done);
   }
-  if (!a.actions || done) {                // reset_world (:35-60); env_wrappers.py:146-152
-    if (a.reset_states) {
-      const double* s = a.reset_states + (size_t)e * (2 + 2 * (M + L));
-      goal[0] = (int)s[0]; goal[1] = (int)s[1];
-      for (int m = 0; m < M; ++m) { ap[m][0] = s[2 + 2 * m]; ap[m][1] = s[3 + 2 * m]; }
-      for (int l = 0; l < L; ++l) { lp[l][0] = s[2 + 2 * (M + l)]; lp[l][1] = s[3 + 2 * (M + l)]; }
-    } else {
-      const uint64_t ctr = *a.rng_counter + (uint64_t)e;
-      double uu[12];
-      for (int q = 0; q < 3; ++q) {
-        const uint4 r = philox4x32_10(make_uint4((uint32_t)ctr, (uint32_t)(ctr >> 32), 0x52454600u + q, 0u),
-                                      make_uint2((uint32_t)a.rng_seed, (uint32_t)(a.rng_seed >> 32)));
-        const uint32_t v[4] = {r.x, r.y, r.z, r.w};
-        for (int j = 0; j < 4; ++j) uu[4 * q + j] = d_mul(d_add((double)v[j], 0.5), 2.3283064365386962890625e-10);
-      }
-      goal[0] = min(L - 1, (int)(uu[10] * L)); goal[1] = min(L - 1, (int)(uu[11] * L));
-      for (int i = 0; i < 2 * M; ++i) ap[i >> 1][i & 1] = d_add(-1.0, d_mul(2.0, uu[i]));
-      for (int i = 0; i < 2 * L; ++i) lp[i >> 1][i & 1] = d_mul(0.8, d_add(-1.0, d_mul(2.0, uu[2 * M + i])));
-    }
-    for (int m = 0; m < M; ++m) { av[m][0] = av[m][1] = 0.0; comm[m] = -1; }   // state.c = zeros
-    step = 0;
-  }
-  for (int m = 0; m < M; ++m)
-    for (int d = 0; d < 2; ++d) { a.apos[((size_t)e * M + m) * 2 + d] = ap[m][d]; a.avel[((size_t)e * M + m) * 2 + d] = av[m][d]; }
-  for (int l = 0; l < L; ++l)
-    for (int d = 0; d < 2; ++d) a.lpos[((size_t)e * L + l) * 2 + d] = lp[l][d];
-  for (int m = 0; m < M; ++m) { a.goal[(size_t)e * M + m] = goal[m]; a.comm[(size_t)e * M + m] = comm[m]; }
-  a.step_count[e] = step;
+  if (!a.actions || done)                  // reset_world; env_wrappers.py:146-152
+    ref_world_reset(w, a.reset_states ? a.reset_states + (size_t)e * kRefResetDoubles : nullptr, a.rng_seed,
+                    a.reset_states ? 0ull : *a.rng_counter + (uint64_t)e);
+  ref_world_store(w, a.apos, a.avel, a.lpos, a.goal, a.comm, a.step_count, e);
   for (int m = 0; m < M; ++m) {
-    float* o = a.obs + ((size_t)e * M + m) * kRefObs;
-    int c = 0;
-    o[c++] = (float)av[m][0]; o[c++] = (float)av[m][1];
-    for (int l = 0; l < L; ++l) { o[c++] = (float)d_sub(lp[l][0], ap[m][0]); o[c++] = (float)d_sub(lp[l][1], ap[m][1]); }
-    for (int k = 0; k < 3; ++k) o[c++] = k == goal[m] ? 0.75f : 0.25f;        // simple_reference.py:46-48
-    for (int k = 0; k < kRefSymbols; ++k) o[c++] = k == comm[1 - m] ? 1.f : 0.f;
+    ref_world_obs(w, m, a.obs + ((size_t)e * M + m) * kRefObs);
     if (a.actions) {
       a.rewards[(size_t)e * M + m] = (float)reward;
       a.dones[(size_t)e * M + m] = done ? 1.f : 0.f;

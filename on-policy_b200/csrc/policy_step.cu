@@ -554,24 +554,64 @@ int rollout_persistent_launch(const NetDev& na, const NetDev& nc, const RolloutA
   return check_launch("rollout_persistent_kernel");
 }
 
-int rollout_closed_launch(const NetDev& na, const NetDev& nc, const ClosedArgs& ca, cudaStream_t st) {
-  const int M = ca.M, L = ca.L;
-  if (!fast_rollout_supported(na) || !fast_rollout_supported(nc) || !ca.r.image[0] || !ca.r.image[1]) { set_error("rollout_closed: needs feed-forward nets (hidden 64, in_dim <= 64) and packed weight images"); return MAPPO_ERR_UNSUPPORTED; }
-  if (M < 1 || M > kMpeMaxAgents || L < 1 || L > kMpeMaxLandmarks || ca.r.E % M != 0) { set_error("rollout_closed: %d agents / %d landmarks / %d rows", M, L, ca.r.E); return MAPPO_ERR_UNSUPPORTED; }
-  if (na.n_heads != 1 || na.head_dim[0] != 5 || na.in_dim != 4 + 2 * L + 4 * (M - 1) || nc.in_dim != M * na.in_dim) { set_error("rollout_closed: policy shapes do not match simple_spread (Discrete(5), obs %d, share_obs %d)", 4 + 2 * L + 4 * (M - 1), M * (4 + 2 * L + 4 * (M - 1))); return MAPPO_ERR_INVALID; }
-  const size_t bytes = closed_smem_bytes(na, nc, M);
-  if (bytes > 227 * 1024) { set_error("rollout_closed: %zu B shared memory", bytes); return MAPPO_ERR_UNSUPPORTED; }
-  auto kern = (M == 3 && L == 3) ? rollout_closed_kernel<3, 3> : rollout_closed_kernel<0, 0>;   // reference default shape
-  static thread_local SmemConfig configured[2] = {};
-  size_t& conf = configured[(M == 3 && L == 3) ? 1 : 0].slot();
-  if (bytes > conf) {
+// raise the kernel's dynamic shared-memory limit once per device
+template <class K>
+static int closed_set_smem(K kern, size_t bytes, SmemConfig& conf) {
+  size_t& c = conf.slot();
+  if (bytes > c) {
     if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) != cudaSuccess)
       return check_launch("rollout_closed: cudaFuncSetAttribute");
-    conf = bytes;
+    c = bytes;
   }
+  return MAPPO_OK;
+}
+
+template <class World>
+static int closed_mlp_launch(const NetDev& na, const NetDev& nc, const ClosedArgs& ca, int M, size_t bytes, cudaStream_t st) {
+  static thread_local SmemConfig conf = {};
+  if (int rc = closed_set_smem(rollout_closed_kernel<World>, bytes, conf)) return rc;
   const int N = ca.r.E / M;
-  kern<<<(N + kCG - 1) / kCG, 64 * kCG * M, bytes, st>>>(na, nc, ca);
+  rollout_closed_kernel<World><<<(N + kCG - 1) / kCG, 64 * kCG * M, bytes, st>>>(na, nc, ca);
   return check_launch("rollout_closed_kernel");
+}
+
+template <class World>
+static int closed_gru_launch(const NetDev& na, const NetDev& nc, const ClosedArgs& ca, const ClosedGruPlan& p, size_t bytes,
+                             cudaStream_t st) {
+  static thread_local SmemConfig conf = {};
+  if (int rc = closed_set_smem(rollout_closed_gru_kernel<World>, bytes, conf)) return rc;
+  rollout_closed_gru_kernel<World><<<2 * p.clusters, 32 * p.warps, bytes, st>>>(na, nc, ca, p.worlds);
+  return check_launch("rollout_closed_gru_kernel");
+}
+
+int rollout_closed_launch(const NetDev& na, const NetDev& nc, const ClosedArgs& ca, cudaStream_t st) {
+  const bool ref = ca.world == MAPPO_WORLD_REFERENCE;
+  const int M = ref ? kRefAgents : ca.M, L = ref ? kRefLandmarks : ca.L;
+  const bool images = ca.r.image[0] && ca.r.image[1];
+  const bool mlp = fast_rollout_supported(na) && fast_rollout_supported(nc);
+  const bool gru = gru_fast_supported(na) && gru_fast_supported(nc) && ca.r.h_actor && ca.r.h_critic;
+  if (!images || !(mlp || gru)) { set_error("rollout_closed: needs two feed-forward or two recurrent nets on the warp-per-row path (hidden 64, in_dim <= 64, <= 32 head outputs; recurrent: with state storage) and packed weight images"); return MAPPO_ERR_UNSUPPORTED; }
+  if (M < 1 || M > kMpeMaxAgents || L < 1 || L > kMpeMaxLandmarks || ca.r.E % M != 0) { set_error("rollout_closed: %d agents / %d landmarks / %d rows", M, L, ca.r.E); return MAPPO_ERR_UNSUPPORTED; }
+  if (ref) {
+    if (na.n_heads != 2 || na.head_dim[0] != 5 || na.head_dim[1] != kRefSymbols || na.in_dim != kRefObs || nc.in_dim != M * kRefObs) { set_error("rollout_closed: policy shapes do not match simple_reference (MultiDiscrete(5, 10), obs %d, share_obs %d)", kRefObs, M * kRefObs); return MAPPO_ERR_INVALID; }
+  } else {
+    const int D = 4 + 2 * L + 4 * (M - 1);
+    if (na.n_heads != 1 || na.head_dim[0] != 5 || na.in_dim != D || nc.in_dim != M * D) { set_error("rollout_closed: policy shapes do not match simple_spread (Discrete(5), obs %d, share_obs %d)", D, M * D); return MAPPO_ERR_INVALID; }
+  }
+  const bool spread33 = !ref && M == 3 && L == 3;             // the reference's default shape: compile-time counts
+  if (mlp) {
+    const size_t bytes = closed_smem_bytes(na, nc, M);
+    if (bytes > 227 * 1024) { set_error("rollout_closed: %zu B shared memory", bytes); return MAPPO_ERR_UNSUPPORTED; }
+    if (ref) return closed_mlp_launch<ReferenceClosedWorld>(na, nc, ca, M, bytes, st);
+    if (spread33) return closed_mlp_launch<SpreadClosedWorld<3, 3>>(na, nc, ca, M, bytes, st);
+    return closed_mlp_launch<SpreadClosedWorld<0, 0>>(na, nc, ca, M, bytes, st);
+  }
+  const ClosedGruPlan p = closed_gru_plan(ca.r.E / M, M, device_sm_count());
+  const size_t bytes = closed_gru_smem_bytes(na, nc, p);
+  if (bytes > 227 * 1024) { set_error("rollout_closed: %zu B shared memory per CTA of the recurrent closed loop > 227 KB", bytes); return MAPPO_ERR_UNSUPPORTED; }
+  if (ref) return closed_gru_launch<ReferenceClosedWorld>(na, nc, ca, p, bytes, st);
+  if (spread33) return closed_gru_launch<SpreadClosedWorld<3, 3>>(na, nc, ca, p, bytes, st);
+  return closed_gru_launch<SpreadClosedWorld<0, 0>>(na, nc, ca, p, bytes, st);
 }
 
 int pack_rollout_launch(const NetDev& n, const float* params, float* image, cudaStream_t st) {

@@ -742,21 +742,6 @@ __host__ __device__ inline TailSmem make_tail_smem(const NetDev& n) {
   return t;
 }
 
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_cta_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// store into the shared memory of CTA `rank` of this cluster, at the address `local` has in this CTA's own window
-__device__ __forceinline__ void st_cluster_f32(const float* local, uint32_t rank, float v) {
-  uint32_t remote;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"((uint32_t)__cvta_generic_to_shared(local)), "r"(rank));
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(remote), "f"(v) : "memory");
-}
-
 __global__ void __cluster_dims__(kTailCtas, 1, 1) __launch_bounds__(kTailThreads, 1) tc_tail_kernel(const TailArgs a) {
   extern __shared__ __align__(16) float tsm[];
   __shared__ float sacc[kTailSubs][kTailUnroll][8][33];

@@ -9,6 +9,7 @@ import os
 MAX_HEADS = 4
 MAX_LAYERS = 2
 GEMM_FP32, GEMM_TF32 = 0, 1
+WORLD_SPREAD, WORLD_REFERENCE = 0, 1          # mappo_rollout_closed_loop_ex
 _LIB_PATH = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "lib", "libmappo_b200.so")
 
 
@@ -80,6 +81,8 @@ _SIGS = {
     "mappo_debug_launch_count": (_i64, []),
     "mappo_rollout_closed_loop": (_i32, [C.POINTER(NetDesc), _P, C.POINTER(NetDesc), _P] + [_P] * 7 + [_P] * 4 +
                                   [_P, _u64, _P, _P, _u64, _P, _i32, _i32, _i32, _i32, _i32, _P]),
+    "mappo_rollout_closed_loop_ex": (_i32, [C.POINTER(NetDesc), _P, C.POINTER(NetDesc), _P] + [_P] * 9 + [_i32] + [_P] * 6 +
+                                     [_P, _u64, _P, _P, _u64, _P, _i32, _i32, _i32, _i32, _i32, _P]),
     "mappo_mpe_spread_step": (_i32, [_P, _P, _P, _P, _P, _P, _u64, _P, _i32, _i32, _i32, _i32, _P, _P, _P, _P, _P]),
     "mappo_mpe_reference_step": (_i32, [_P, _P, _P, _P, _P, _P, _P, _P, _u64, _P, _i32, _i32, _P, _P, _P, _P, _P]),
     "mappo_minibatch_stats_batch": (_i32, [_P, _P, _P, _i64, _i32, _i32, _P, _P]),

@@ -9,8 +9,9 @@ and -- in "host" RNG mode -- the reference's sampling noise / permutations), one
 The rollout kernels write values / actions / log-probs / rnn states STRAIGHT into the storage slots.  Three collect modes:
   * staged feed, persistent (default): all T steps + inserts + the bootstrap value in ONE launch (mappo_rollout_persistent),
   * staged feed, per step: T x (mappo_policy_step + mappo_env_insert)  (MAPPO_B200_PERSISTENT_ROLLOUT=0),
-  * closed loop (device_env=DeviceSpreadEnv): the MPE simple_spread worlds are stepped on the device between policy and
-    insert -- inside one persistent kernel (mappo_rollout_closed_loop) or as one extra launch per step.
+  * closed loop (device_env=DeviceSpreadEnv or DeviceReferenceEnv): the MPE worlds are stepped on the device between policy
+    and insert -- inside one persistent kernel (mappo_rollout_closed_loop_ex; feed-forward and GRU policies, default) or as
+    one extra launch per step (MAPPO_B200_PERSISTENT_ROLLOUT=0).
 """
 from __future__ import annotations
 
@@ -64,7 +65,7 @@ def warp_per_row_rollout(*descs) -> bool:
     """True when every net qualifies for the warp-per-row rollout kernels: hidden 64, in_dim <= 64 and at most 32 head
     outputs (csrc/rollout_mlp.cuh fast_rollout_supported, csrc/rollout_gru.cuh gru_fast_supported).  The persistent
     rollout takes that path only when BOTH nets qualify; otherwise it runs the 32-row tile kernels, which read share_obs
-    from its own staging buffer, and mappo_rollout_closed_loop is not built at all."""
+    from its own staging buffer, and the one-launch closed loop (mappo_rollout_closed_loop_ex) is not built at all."""
     return all(d.hidden == 64 and d.in_dim <= 64 and sum(d.head_dim[k] for k in range(d.n_heads)) <= 32 for d in descs)
 
 
@@ -74,8 +75,10 @@ class RolloutEngine:
         """share_obs_from_obs: the env's share_obs is the concatenation of the obs of the agents of a rollout thread
         (what the MPE runner builds on the host, mpe_runner.py:133-135): only obs is staged / uploaded and the critic
         reads its rows from it on the device (feed-forward policies, persistent rollout).
-        device_env: a mappo_b200.mpe_env.DeviceSpreadEnv -- CLOSED LOOP: every collect step is policy_step -> env step ->
-        insert on the device (no staged feed, no upload; the env writes into the staging buffers the insert reads)."""
+        device_env: a mappo_b200.mpe_env.DeviceSpreadEnv or DeviceReferenceEnv -- CLOSED LOOP: every collect step is
+        policy_step -> env step -> insert on the device (no staged feed, no upload).  By default the whole collect is one launch
+        with the worlds inside the rollout kernel; with MAPPO_B200_PERSISTENT_ROLLOUT=0 the env writes into the staging buffers
+        the per-step insert reads."""
         self.args, self.policy, self.trainer, self.buffer = args, policy, trainer, buffer
         self.dev = policy.device
         self.rng = rng
@@ -92,7 +95,7 @@ class RolloutEngine:
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=self.dev)
         import os
         self.env = device_env
-        self.env_reset_states = None        # optional [T, N, 2 (M + L)] float64: injected episode starts (parity tests)
+        self.env_reset_states = None        # optional [T, N, reset doubles per world] float64: injected episode starts (parity tests)
         want_persistent = os.environ.get("MAPPO_B200_PERSISTENT_ROLLOUT", "1") == "1"
         # hidden >= 128 nets run the layer-by-layer GEMM pipeline per step (the persistent kernels keep weights in shared memory)
         self.big = bool(self.lib.mappo_big_net(C.byref(policy.actor.desc)))
@@ -102,10 +105,10 @@ class RolloutEngine:
                 raise NotImplementedError("closed-loop device env with hidden >= 128 nets")
             want_persistent = False
         self.persistent_rollout = want_persistent and device_env is None
-        # closed loop as ONE launch (mappo_rollout_closed_loop): feed-forward policies whose nets both take the warp-per-row
-        # path (a wider critic, e.g. 4-agent simple_spread's share_obs of 96, steps the env per step instead)
+        # closed loop as ONE launch (mappo_rollout_closed_loop_ex): feed-forward or GRU policies whose nets both take the
+        # warp-per-row path (a wider critic, e.g. 4-agent simple_spread's share_obs of 96, steps the env per step instead)
         fast = warp_per_row_rollout(policy.actor.desc, policy.critic.desc)
-        self.closed_persistent = want_persistent and device_env is not None and not self.recurrent and fast
+        self.closed_persistent = want_persistent and device_env is not None and fast
         if device_env is not None and (device_env.N * device_env.M != E or device_env.obs_dim != self.Do
                                        or device_env.share_dim != self.Ds):
             raise ValueError("device_env does not match the rollout storage (rows / obs_dim / share_obs_dim)")
@@ -260,15 +263,19 @@ class RolloutEngine:
             ptr(self.d_noise), self.seed, ptr(pol.rng_offset), self.T, self.E, stream_ptr()))
 
     def _rollout_closed(self):
-        """Closed loop, all T steps + the bootstrap value as ONE launch (policy -> world step -> insert inside the kernel)."""
+        """Closed loop, all T steps + the bootstrap value as ONE launch (policy -> world step -> insert inside the kernel); the
+        world kind comes from the env (simple_spread / simple_reference)."""
         b, pol, lib, env = self.buffer, self.policy, self.lib, self.env
         rs = self.env_reset_states
-        check(lib.mappo_rollout_closed_loop(
+        rec = self.recurrent
+        ref = env.WORLD == _lib.WORLD_REFERENCE
+        check(lib.mappo_rollout_closed_loop_ex(
             C.byref(pol.actor.desc), ptr(self.img_actor), C.byref(pol.critic.desc), ptr(self.img_critic),
-            ptr(b.obs), ptr(b.share_obs), ptr(b.masks), ptr(b.value_preds), ptr(b.actions), ptr(b.action_log_probs),
-            ptr(b.rewards), ptr(env.apos), ptr(env.avel), ptr(env.lpos), ptr(env.step_count),
-            ptr(rs) if rs is not None else None, env.seed, ptr(env.rng_counter), ptr(self.d_noise), self.seed,
-            ptr(pol.rng_offset), self.T, self.E, env.M, env.L, env.EP, stream_ptr()))
+            ptr(b.obs), ptr(b.share_obs), ptr(b.rnn_states) if rec else None, ptr(b.rnn_states_critic) if rec else None,
+            ptr(b.masks), ptr(b.value_preds), ptr(b.actions), ptr(b.action_log_probs), ptr(b.rewards), env.WORLD,
+            ptr(env.apos), ptr(env.avel), ptr(env.lpos), ptr(env.goal) if ref else None, ptr(env.comm) if ref else None,
+            ptr(env.step_count), ptr(rs) if rs is not None else None, env.seed, ptr(env.rng_counter), ptr(self.d_noise),
+            self.seed, ptr(pol.rng_offset), self.T, self.E, env.M, env.L, env.EP, stream_ptr()))
 
     def _returns(self):
         b, lib, st, T = self.buffer, self.lib, stream_ptr(), self.T

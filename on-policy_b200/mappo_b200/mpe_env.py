@@ -5,6 +5,8 @@ mappo_mpe_spread_step / mappo_mpe_reference_step.
 buffers the rollout kernels consume -- a collect step then has no host round trip (the reference pays a SubprocVecEnv pipe
 round trip plus NumPy physics per step, envs/env_wrappers.py:257-266).  `DeviceSpreadVecEnv` wraps it in the reference's
 vec-env interface (reset() / step(one-hot actions) -> obs, rews, dones, infos as NumPy) so the unchanged runner can use it.
+Either env can also be stepped inside the one-launch closed rollout loop (engine.RolloutEngine(device_env=...)), which reads
+and writes the same state tensors.
 """
 from __future__ import annotations
 
@@ -19,6 +21,8 @@ from .core import stream_ptr
 
 
 class DeviceSpreadEnv:
+    WORLD = _lib.WORLD_SPREAD              # world kind of the one-launch closed loop (engine.RolloutEngine)
+
     def __init__(self, n_envs: int, num_agents: int = 3, num_landmarks: int = 3, episode_length: int = 25,
                  device="cuda", seed: int = 1):
         self.lib = _lib.load()
@@ -95,6 +99,7 @@ class DeviceReferenceEnv:
     """N `simple_reference` worlds on the device (mappo_mpe_reference_step): 2 agents, 3 landmarks, 10 symbols;
     actions [N*2, 2] = (move, symbol) as the policy stores a MultiDiscrete sample; obs [N*2, 21]."""
     M, L, DIM_C = 2, 3, 10
+    WORLD = _lib.WORLD_REFERENCE
 
     def __init__(self, n_envs: int, episode_length: int = 25, device="cuda", seed: int = 1):
         self.lib = _lib.load()
